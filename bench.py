@@ -1,6 +1,6 @@
 """bench.py -- particle-pair interactions/s on the 3D WCSPH dam break.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...      # the CPU arm (oracle, all threads)
 
@@ -560,6 +560,33 @@ def run_rings(args, emit, rank=0, local_rank=0, world=1):
     })
 
 
+DUMP_FIELDS = ('x', 'y', 'z', 'u', 'v', 'w', 'rho', 'p', 'arho', 'au', 'av', 'aw')
+DUMP_SAMPLE = 131072     # particles per array: 3 arrays x 13 fp64 columns stay under 64 MB
+
+
+def dump_outputs(be, out_dir):
+    """--dump-outputs: what a caller of the timed steps receives after the last of them --
+    every array's real particles, pulled from the device, as DIR/<array>_<field>.npy
+    (float64) with DIR/<array>_gid.npy naming the particles.  Rows are in gid order, so the
+    files do not depend on how the device orders particles; an array of more than
+    DUMP_SAMPLE particles is sampled at fixed, seeded positions of that order.  The host
+    mirrors are left as they are (the e2e loop pushes them)."""
+    from pysph_b200 import _lib
+    os.makedirs(out_dir, exist_ok=True)
+    for i, pa in enumerate(be.particle_arrays):
+        n = be.sizes(i)[1]
+        gid = np.empty(n, dtype=np.uint32)
+        be.ctx.call('b200sph_pull_u32', i, _lib.INT_PROP_IDS['gid'], gid.ctypes.data, 0, n)
+        rows = np.argsort(gid, kind='stable')
+        if n > DUMP_SAMPLE:
+            rows = rows[np.sort(np.random.RandomState(i).choice(n, DUMP_SAMPLE, replace=False))]
+        np.save(os.path.join(out_dir, '%s_gid.npy' % pa.name), gid[rows].astype(np.float64))
+        for f in DUMP_FIELDS:
+            col = np.empty(n, dtype=np.float64)
+            be.ctx.call('b200sph_pull_f64', i, be.prop_ids[i][f], col.ctypes.data, 0, n)
+            np.save(os.path.join(out_dir, '%s_%s.npy' % (pa.name, f)), col[rows])
+
+
 def pinned_arrays(pas):
     """Re-home every property of the ParticleArrays in pinned host memory."""
     import torch
@@ -597,11 +624,21 @@ def main():
     ap.add_argument('--no-extras', action='store_true',
                     help='skip the sub-records of BASELINE configs[3] / [4] (and configs[2] as '
                          'quoted at N = 8) appended to the dam-break line')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='single-GPU dam break: after the timed steps, write the particle fields '
+                         'of their last step to DIR/<array>_<field>.npy (float64, gid order, at '
+                         'most %d particles per array, sampled with a fixed seed) to compare '
+                         'two builds output for output' % DUMP_SAMPLE)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
 
     rank = int(os.environ.get('RANK', '0'))
     local_rank = int(os.environ.get('LOCAL_RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
+    if args.dump_outputs and (args.impl != 'b200' or args.workload != 'dam_break' or world > 1):
+        ap.error('--dump-outputs: only the single-GPU dam break (--impl b200 --workload '
+                 'dam_break --gpus 1) writes its outputs')
     if world == 1 and args.gpus > 1:
         print('bench.py: --gpus %d needs torch.distributed.run with '
               '--nproc-per-node %d' % (args.gpus, args.gpus), file=sys.stderr)
@@ -851,6 +888,9 @@ def run_dam_break(args, rank, local_rank, world):
         return e0.elapsed_time(e1), be.stats(), cpu_ms, first_line
 
     ms_total, st, cpu_enqueue_ms, n_s0 = timed_steps()
+    # the first K timed steps, not a re-measured region: the dump depends on the arguments only
+    if args.dump_outputs:
+        dump_outputs(be, args.dump_outputs)
     if os.environ.get('B200SPH_PM_PROFILE') and pm is None:
         sys.stderr.write('[pm-profile rank 0] per step: cpu_loop %.3f ms\n' % (cpu_enqueue_ms / K))
     if pm is not None and getattr(pm, '_prof', None) is not None:

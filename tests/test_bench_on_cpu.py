@@ -52,13 +52,8 @@ CONTRACT = ['metric', 'value', 'unit', 'n_gpus', 'steps', 'warmup', 'ms_per_step
             'e2e', 'gpu_launches', 'roofline', 'cpu_baseline']
 
 
-@pytest.mark.parametrize('argv', [
-    ['--dx', '0.08'],
-    ['--workload', 'taylor_green', '--nx', '10'],
-    ['--workload', 'rings', '--dx', '0.0025', '--lz', '0.0075'],
-], ids=['dam_break', 'taylor_green', 'rings'])
-def test_bench_gpu_arm_on_the_emulated_library(emulated_library, fake_cuda, monkeypatch,  # noqa: F811
-                                               capfd, argv):
+def _bench_line(monkeypatch, capfd, argv):
+    """bench.main() in this process; returns its one JSON line"""
     sys.path.insert(0, ROOT)
     bench = importlib.import_module('bench')
     monkeypatch.setattr(sys, 'argv', ['bench.py', '--steps', '3', '--warmup', '3',
@@ -74,7 +69,17 @@ def test_bench_gpu_arm_on_the_emulated_library(emulated_library, fake_cuda, monk
     out = capfd.readouterr().out
     lines = [ln for ln in out.splitlines() if ln.startswith('{')]
     assert len(lines) == 1, out[-2000:]
-    d = json.loads(lines[0])
+    return json.loads(lines[0])
+
+
+@pytest.mark.parametrize('argv', [
+    ['--dx', '0.08'],
+    ['--workload', 'taylor_green', '--nx', '10'],
+    ['--workload', 'rings', '--dx', '0.0025', '--lz', '0.0075'],
+], ids=['dam_break', 'taylor_green', 'rings'])
+def test_bench_gpu_arm_on_the_emulated_library(emulated_library, fake_cuda, monkeypatch,  # noqa: F811
+                                               capfd, argv):
+    d = _bench_line(monkeypatch, capfd, argv)
     for k in CONTRACT:
         assert k in d, k
     assert d['unit'] == 'pairs/s' and d['n_gpus'] == 1 and d['steps'] == 3 and d['warmup'] == 3
@@ -89,6 +94,34 @@ def test_bench_gpu_arm_on_the_emulated_library(emulated_library, fake_cuda, monk
     assert r['bound'] == 'hbm' and r['unit'] == 'GB/s' and r['peak'] > 0
     c = d['cpu_baseline']
     assert c['kind'] == 'port' and c['cores'] == 1 and c['value'] > 0 and c['sample']
+
+
+def test_bench_dump_outputs_on_the_emulated_library(emulated_library, fake_cuda,  # noqa: F811
+                                                    monkeypatch, capfd, tmp_path):
+    """--dump-outputs DIR: the same arguments write the same files (float64, rows in gid order,
+    arrays above the sample size sampled), and --steps sets how far the dumped state got."""
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    bench = importlib.import_module('bench')
+    monkeypatch.setattr(bench, 'DUMP_SAMPLE', 200)
+    base = ['--dx', '0.08', '--no-cpu', '--no-developed', '--no-extras']
+    runs = {}
+    for tag, steps in (('a', 3), ('b', 3), ('c', 4)):
+        d = _bench_line(monkeypatch, capfd, base + ['--steps', str(steps),
+                                                    '--dump-outputs', str(tmp_path / tag)])
+        assert d['steps'] == steps
+        runs[tag] = dict((p.name[:-4], np.load(p)) for p in (tmp_path / tag).iterdir())
+    a = runs['a']
+    names = ('fluid', 'boundary', 'obstacle')
+    assert sorted(a) == sorted('%s_%s' % (n, f) for n in names for f in ('gid',) + bench.DUMP_FIELDS)
+    for k, v in a.items():
+        assert v.dtype == np.float64 and v.ndim == 1 and np.all(np.isfinite(v)), k
+        assert np.array_equal(v, runs['b'][k]), k
+    for n in names:
+        g = a[n + '_gid']
+        assert 0 < len(g) <= 200 and np.all(np.diff(g) > 0), n
+    assert len(a['fluid_gid']) == 200            # the fluid is larger than the sample
+    assert not np.array_equal(a['fluid_w'], runs['c']['fluid_w'])
 
 
 def _rank_main(rank, world, port, so, argv, q):

@@ -79,7 +79,7 @@ def _worker(rank, world, port, q):
         dist.destroy_process_group()
 
 
-@pytest.mark.skipif(_ngpus() < 2, reason='needs >= 2 GPUs (run under gpurun --gpus 2)')
+@pytest.mark.skipif(_ngpus() < 2, reason='needs >= 2 GPUs')
 @pytest.mark.parametrize('world', [2])
 def test_slab_decomposition_matches_single_gpu(world):
     import torch.multiprocessing as mp

@@ -2,7 +2,7 @@
 `k_column_counts` and `SlabParallelManager._recut`.  Also covered on the host emulation of
 the library (tests/test_library_on_cpu.py: slab decomposition with lb_freq=2 on 3 ranks)
 and with the numpy test double (tests/test_parallel_gloo.py: test_slab_recut_gloo).  The
-2-GPU test needs `gpurun --gpus 2` (skipped on a 1-GPU lease)."""
+2-GPU test skips on a machine with one GPU."""
 import numpy as np
 import pytest
 
@@ -74,7 +74,7 @@ def test_recut_slabs_match_single_gpu():
     from pysph_b200 import geometry as geo, parallel
     import test_gpu_multi as M
     if torch.cuda.device_count() < 2:
-        pytest.skip('needs >= 2 GPUs (run under gpurun --gpus 2)')
+        pytest.skip('needs >= 2 GPUs')
     world = 2
     params = geo.dam_break_3d_params(M.DX)
     pas = geo.dam_break_3d_particles(dx=M.DX)

@@ -2,7 +2,7 @@
 16-field ghost message, the 30-field migration message and group 1 on a two-support halo.
 The same comparison runs on the library emulation over gloo with 3 ranks
 (tests/test_library_on_cpu.py::test_rings_slab_decomposition_on_the_emulated_library);
-here it runs on 2 GPUs with the peer-memory refresh; needs >= 2 GPUs (gpurun --gpus 2),
+here it runs on 2 GPUs with the peer-memory refresh and skips on a machine with one GPU;
 the layout tests run on one."""
 import os
 
@@ -39,7 +39,7 @@ def _worker(rank, world, port, q):
         dist.destroy_process_group()
 
 
-@pytest.mark.skipif(_ngpus() < 2, reason='needs >= 2 GPUs (run under gpurun --gpus 2)')
+@pytest.mark.skipif(_ngpus() < 2, reason='needs >= 2 GPUs')
 def test_rings_slabs_match_single_gpu():
     import torch.multiprocessing as mp
     import pysph_b200 as pb
@@ -85,7 +85,6 @@ def test_elastic_halo_and_migration_layout(gpu_device):
     """One GPU: with elastic-dynamics arrays b200sph_halo_layout reports 16 / 30 fields, the
     ghost message is x y z u v w rho h m s00 s01 s02 s11 s12 s22 cs, the migration message
     the 16 fp64 state properties, gid, s00..s22, s000..s220, cs -- field-major, exact."""
-    import torch
     import pysph_b200 as pb
     from pysph_b200.parallel import DeviceHaloOps
     rs = np.random.RandomState(5)
@@ -101,8 +100,6 @@ def test_elastic_halo_and_migration_layout(gpu_device):
     cs32 = ref['cs'].astype(np.float32).astype(np.float64)      # cs is fp32 on the device
     be = pb.B200Backend([a, b], extra_capacity=2000)
     ops = DeviceHaloOps(be, 0)
-    if not torch.cuda.is_available():          # the library emulation: device memory is host memory
-        ops.device = torch.device('cpu')
     assert (ops.halo_nf, ops.migrate_nf) == (16, 30)
     lo, hi = 1.0, 1.6
     buf = ops.new_buffer(16 * n)

@@ -179,6 +179,8 @@ def _id(t):
 
 
 def _call(t, emulated_library):
+    import torch
+    from pysph_b200 import parallel
     mod = __import__(t[0])
     fn = getattr(mod, t[1])
     fn = getattr(fn, '__wrapped__', fn)
@@ -187,11 +189,18 @@ def _call(t, emulated_library):
         import pathlib
         import tempfile
         kw['tmp_path'] = pathlib.Path(tempfile.mkdtemp())
-    if 'monkeypatch' in kw:
-        with pytest.MonkeyPatch.context() as mp:
+    init = parallel.DeviceHaloOps.__init__
+
+    def host_init(self, backend, device):
+        init(self, backend, 0)
+        self.device = torch.device('cpu')
+    with pytest.MonkeyPatch.context() as mp:
+        # halo buffers in host memory: under the emulation device memory IS host memory, also
+        # on a machine where torch sees a GPU
+        mp.setattr(parallel.DeviceHaloOps, '__init__', host_init)
+        if 'monkeypatch' in kw:
             kw['monkeypatch'] = mp
-            return fn(emulated_library, **kw)
-    return fn(emulated_library, **kw)
+        return fn(emulated_library, **kw)
 
 
 @pytest.mark.parametrize('t', FAST, ids=_id)
