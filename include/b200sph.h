@@ -307,6 +307,13 @@ int b200sph_ferrari_h(b200sph_ctx *ctx, int arr, double hdx, int dim,
  * (dest, source) loops); counting costs one extra atomic per warp. */
 int b200sph_pair_pass(b200sph_ctx *ctx, const b200sph_pair_program *prog,
                       int64_t *pairs_out);
+/* on != 0: no program or stepper run on this context writes h or m on the device (host pushes
+ * may still change them).  With it, a pair pass of the WCSPH Group may gather one 32-byte record
+ * per neighbour instead of 48 bytes when every particle has the same h, m is uniform within each
+ * source class and every source array's equation of state is Tait with gamma = 7 (at most two
+ * source classes, no ghosts; env B200SPH_PAIR_R32=0 turns it off).  b200sph_ferrari_h and a
+ * generic launch that writes h switch it off.  Default off. */
+int b200sph_set_hm_static(b200sph_ctx *ctx, int on);
 /* Group(start_idx, stop_idx) (equation.py:448-520; D_START_IDX / NP_DEST of the generated
  * loop, acceleration_eval_cython_helper.py:259-284): the NEXT b200sph_pair_pass only touches
  * the destinations [start, stop) of array `arr` (indices into the array; stop = -1: to the end,
@@ -576,6 +583,9 @@ int b200sph_column_counts(b200sph_ctx *ctx, int arr, double x0, double inv_width
 
 /* ---- bookkeeping -------------------------------------------------------- */
 int b200sph_get_stats(b200sph_ctx *ctx, b200sph_stats *out);
+/* pair passes since the last reset_stats that ran the 32-byte-record list kernel
+ * (b200sph_set_hm_static); kept out of b200sph_stats so that its layout stays */
+int b200sph_get_pair_r32_launches(b200sph_ctx *ctx, int64_t *out);
 int b200sph_reset_stats(b200sph_ctx *ctx);
 /* per-phase CUDA-event timing: 0 off, 1 every phase (ms_nnps, ms_pair, ms_other),
  * 2 the pair kernels only (ms_pair; two events per pair pass instead of ~25 per

@@ -147,6 +147,7 @@ SIGNATURES = {
     'b200sph_eos': (C.c_int, [_ctx_p, C.c_int, C.c_int, C.c_double, C.c_double,
                               C.c_double, C.c_double, C.c_int]),
     'b200sph_ferrari_h': (C.c_int, [_ctx_p, C.c_int, C.c_double, C.c_int, C.c_int]),
+    'b200sph_set_hm_static': (C.c_int, [_ctx_p, C.c_int]),
     'b200sph_pair_pass': (C.c_int, [_ctx_p, C.POINTER(PairProgram),
                                     C.POINTER(_i64)]),
     'b200sph_set_dest_range': (C.c_int, [_ctx_p, C.c_int, _i64, _i64]),
@@ -216,6 +217,7 @@ SIGNATURES = {
                                         C.c_void_p]),
     'b200sph_get_stats': (C.c_int, [_ctx_p, C.POINTER(Stats)]),
     'b200sph_reset_stats': (C.c_int, [_ctx_p]),
+    'b200sph_get_pair_r32_launches': (C.c_int, [_ctx_p, C.POINTER(C.c_int64)]),
     'b200sph_set_profiling': (C.c_int, [_ctx_p, C.c_int]),
 }
 

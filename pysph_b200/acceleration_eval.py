@@ -46,6 +46,12 @@ class B200AccelerationEval(object):
         # properties the generated kernels use beyond the pool's own
         for name in self._generic_props.user:
             self.backend.add_user_property(name)
+        # h and m stay what the host pushed unless an op writes them (UpdateSmoothingLengthFerrari,
+        # a translated equation storing to h or m); with several evaluators on one backend, one
+        # such op anywhere decides.  The library then may use uniform h / m as constants.
+        self.backend.hm_static = getattr(self.backend, 'hm_static', True) and \
+            not _writes_h_or_m(self.ops)
+        self.ctx.call('b200sph_set_hm_static', int(self.backend.hm_static))
         self._range = None
         self.nnps = None
         self.count_pairs = False
@@ -162,3 +168,18 @@ class B200AccelerationEval(object):
                          gg.real_only, float(t), float(dt), gg.write_flags)
             for eq in reduces:           # host side, after post_loop (mako:127-130)
                 eq.reduce(self.particle_arrays[d], t, dt)
+
+
+def _writes_h_or_m(ops):
+    """Whether an op of the list (nested ones included) stores to h or m on the device."""
+    for op in ops:
+        kind = op[0]
+        if kind == 'ferrari':
+            return True
+        if kind == 'generic' and set(op[1].writes) & {'h', 'm'}:
+            return True
+        if kind == 'cond' and _writes_h_or_m(op[2]):
+            return True
+        if kind == 'iterate' and _writes_h_or_m(op[4]):
+            return True
+    return False

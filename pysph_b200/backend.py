@@ -244,7 +244,11 @@ class B200Backend(object):
     def stats(self):
         s = _lib.Stats()
         self.ctx.call('b200sph_get_stats', C.byref(s))
-        return dict((k, getattr(s, k)) for k, _ in s._fields_)
+        out = dict((k, getattr(s, k)) for k, _ in s._fields_)
+        n = C.c_int64(0)
+        self.ctx.call('b200sph_get_pair_r32_launches', C.byref(n))
+        out['pair_r32_launches'] = n.value
+        return out
 
     def synchronize(self):
         self.ctx.call('b200sph_synchronize')

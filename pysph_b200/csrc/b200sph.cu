@@ -202,10 +202,12 @@ struct b200sph_ctx {
     uint32_t *perm_tmp = nullptr, *perm = nullptr, *skey = nullptr, *rank = nullptr;
     float4 *A = nullptr, *B = nullptr, *C = nullptr;
     float4 *AB = nullptr;  // {A, B} interleaved (32 B = one sector per particle) for the list consumer's 256-bit gathers
+    float4 *R = nullptr;   // 32-byte source records of the R32 list kernel (PairArgs.R)
     int64_t n_sorted = 0;
     bool state_packed = false;
     int force_kernel = 0;       // 0 lists (default), 1 warp kernel (env B200SPH_PAIR_KERNEL)
     int pair_minb = 7;          // resident CTAs per SM k_pair_list is compiled for (env B200SPH_PAIR_MINB: 6, 7, 8)
+    int pair_minb_r32 = 8;      // ... its R32 form (7 or 8; the same env sets both): 8 measured 5 % faster than 7
     bool zorder = false;        // cell rows along the Z-curve of (cy, cz) (env B200SPH_ZORDER; measured: profiles/)
     bool pair_spec = true;      // use the WCSPH-only variant of k_pair_list when the program allows (env B200SPH_PAIR_SPEC)
     // persistent neighbour lists
@@ -253,6 +255,16 @@ struct b200sph_ctx {
     std::atomic<bool> snap_open{false};   // taken by the time loop, released by the output thread
     cudaEvent_t tc_evt[2] = {nullptr, nullptr};
     bool h_dirty = true;        // h changed since the last update_domain reduction
+    // the 32-byte-record list kernel (k_pair_list<..., R32>, env B200SPH_PAIR_R32): allowed by the
+    // caller (b200sph_set_hm_static), and the per-array h / m extrema it needs, re-reduced when
+    // h or m may have changed (uni_dirty)
+    bool pair_r32 = true;
+    bool hm_static = false;
+    bool uni_dirty = true;
+    double uni_h[B200SPH_MAX_ARRAYS][2], uni_m[B200SPH_MAX_ARRAYS][2];   // (min, max) over the real particles
+    long long *uni_red = nullptr;   // device scratch of k_uni_minmax
+    unsigned r32_cls = 0;       // bit a: array a is source class 1 in R (what the state packers write)
+    int64_t n_pair_r32 = 0;     // pair passes that ran it (since reset_stats)
     unsigned *red_u32 = nullptr, *red_u32_host = nullptr;
     int64_t n_full_builds = 0, n_light_updates = 0, n_list_builds = 0;
 
@@ -554,6 +566,7 @@ static int pool_layout(b200sph_ctx *ctx, const int64_t *new_cap)
     if (ctx->B) cudaFree(ctx->B);
     if (ctx->C) cudaFree(ctx->C);
     if (ctx->AB) cudaFree(ctx->AB);
+    if (ctx->R) cudaFree(ctx->R);
     if (ctx->A0) cudaFree(ctx->A0);
     if (ctx->Dv) cudaFree(ctx->Dv);
     if (ctx->PT) cudaFree(ctx->PT);
@@ -570,6 +583,7 @@ static int pool_layout(b200sph_ctx *ctx, const int64_t *new_cap)
     CU(cudaMalloc((void **)&ctx->B, 16 * (size_t)alloc));
     CU(cudaMalloc((void **)&ctx->C, 16 * (size_t)alloc));
     CU(cudaMalloc((void **)&ctx->AB, 32 * (size_t)alloc));
+    CU(cudaMalloc((void **)&ctx->R, 32 * (size_t)alloc));
     CU(cudaMalloc((void **)&ctx->A0, 16 * (size_t)alloc));
     CU(cudaMalloc((void **)&ctx->Dv, 16 * (size_t)alloc));
     CU(cudaMalloc((void **)&ctx->PT, 8 * (size_t)alloc));
@@ -578,7 +592,7 @@ static int pool_layout(b200sph_ctx *ctx, const int64_t *new_cap)
     CU(cudaMalloc((void **)&ctx->stype, (size_t)alloc));
     ctx->lists_valid = false;
     ctx->topo_dirty = true;
-    ctx->h_dirty = true;
+    ctx->h_dirty = ctx->uni_dirty = true;
     CU(cudaMalloc((void **)&ctx->flag_a, 4 * (size_t)(alloc + 1)));
     CU(cudaMalloc((void **)&ctx->flag_b, 4 * (size_t)(alloc + 1)));
     ctx->flag_cap = alloc + 1;
@@ -753,9 +767,10 @@ int b200sph_create(int device, b200sph_ctx **out)
             return -3;
         }
     }
-    if (const char *e = getenv("B200SPH_PAIR_MINB")) ctx->pair_minb = atoi(e);
+    if (const char *e = getenv("B200SPH_PAIR_MINB")) ctx->pair_minb = ctx->pair_minb_r32 = atoi(e);
     if (const char *e = getenv("B200SPH_FUSE")) ctx->fuse = atoi(e) != 0;
     if (const char *e = getenv("B200SPH_PAIR_SPEC")) ctx->pair_spec = atoi(e) != 0;
+    if (const char *e = getenv("B200SPH_PAIR_R32")) ctx->pair_r32 = atoi(e) != 0;
     if (const char *e = getenv("B200SPH_ZORDER")) ctx->zorder = atoi(e) != 0;
     if (const char *e = getenv("B200SPH_PROACTIVE")) ctx->proactive = atoi(e) != 0;
     if (const char *e = getenv("B200SPH_PUSH_FIRST")) ctx->push_first = atoi(e) != 0;
@@ -793,7 +808,7 @@ int b200sph_destroy(b200sph_ctx *ctx)
     cudaFree(ctx->ptype);
     cudaFree(ctx->key_of); cudaFree(ctx->off_in); cudaFree(ctx->cell_cnt); cudaFree(ctx->cell_start);
     cudaFree(ctx->blk_sums); cudaFree(ctx->perm_tmp); cudaFree(ctx->perm); cudaFree(ctx->skey);
-    cudaFree(ctx->rank); cudaFree(ctx->A); cudaFree(ctx->B); cudaFree(ctx->C); cudaFree(ctx->AB);
+    cudaFree(ctx->rank); cudaFree(ctx->A); cudaFree(ctx->B); cudaFree(ctx->C); cudaFree(ctx->AB); cudaFree(ctx->R); cudaFree(ctx->uni_red);
     cudaFree(ctx->red); cudaFreeHost(ctx->red_host); cudaFree(ctx->counter);
     cudaFreeHost(ctx->counter_host); cudaFree(ctx->stage_buf); cudaFree(ctx->flag_a);
     cudaFree(ctx->flag_b); cudaFree(ctx->A0); cudaFree(ctx->lst); cudaFree(ctx->cnt);
@@ -882,7 +897,7 @@ int b200sph_add_array(b200sph_ctx *ctx, const char *name, int64_t n, int64_t n_r
     ctx->ptype_dirty = true;
     ctx->grid_valid = false, ctx->packed_valid = false;
     ctx->topo_dirty = true;
-    ctx->h_dirty = true;
+    ctx->h_dirty = ctx->uni_dirty = true;
     return a;
 }
 
@@ -903,7 +918,7 @@ int b200sph_resize_array(b200sph_ctx *ctx, int arr, int64_t n, int64_t n_real)
     ctx->ptype_dirty = true;
     ctx->grid_valid = false, ctx->packed_valid = false;
     ctx->topo_dirty = true;
-    ctx->h_dirty = true;
+    ctx->h_dirty = ctx->uni_dirty = true;
     return 0;
 }
 
@@ -990,7 +1005,8 @@ int b200sph_push_f64(b200sph_ctx *ctx, int arr, int prop, const double *host, in
     if (!ctx->async_copies) CU(cudaStreamSynchronize(ctx->stream));
     // new positions / smoothing lengths for the SAME particles: the next nnps_update
     // measures the drift against the current neighbour build and reuses it if it can
-    if (prop == B200SPH_H) { ctx->domain_valid = false; ctx->h_dirty = true; }
+    if (prop == B200SPH_H) { ctx->domain_valid = false; ctx->h_dirty = ctx->uni_dirty = true; }
+    if (prop == B200SPH_M) ctx->uni_dirty = true;
     if (prop <= B200SPH_Z || prop == B200SPH_H) ctx->grid_valid = false, ctx->packed_valid = false;
     ctx->state_packed = false;
     return 0;
@@ -1169,7 +1185,7 @@ int b200sph_set_kernel(b200sph_ctx *ctx, int kernel, int dim)
     ctx->domain_valid = false;
     ctx->grid_valid = false, ctx->packed_valid = false;
     ctx->topo_dirty = true;
-    ctx->h_dirty = true;
+    ctx->h_dirty = ctx->uni_dirty = true;
     return 0;
 }
 
@@ -1317,7 +1333,7 @@ static int nnps_light_update(b200sph_ctx *ctx)
         if (ctx->packed_valid) return 1;   // nnps_drift_device packed them, halo_overwrite_all kept the ghosts current
         k_pack_pos_light<<<(unsigned)cdiv(ctx->n_sorted, 256), 256, 0, ctx->stream>>>(
             ctx->f64[B200SPH_X], ctx->f64[B200SPH_Y], ctx->f64[B200SPH_Z], ctx->f64[B200SPH_H], ctx->perm, ctx->skey,
-            ctx->n_sorted, ctx->G, ctx->A0, ctx->A, ctx->AB, ctx->red_u32);
+            ctx->n_sorted, ctx->G, ctx->A0, ctx->A, ctx->AB, ctx->R, ctx->red_u32);
         LAUNCH_CHECK();
         return 1;
     }
@@ -1325,7 +1341,7 @@ static int nnps_light_update(b200sph_ctx *ctx)
         CU(cudaMemsetAsync(ctx->red_u32, 0, 4 * sizeof(unsigned), ctx->stream));
         k_pack_pos_light<<<(unsigned)cdiv(ctx->n_sorted, 256), 256, 0, ctx->stream>>>(
             ctx->f64[B200SPH_X], ctx->f64[B200SPH_Y], ctx->f64[B200SPH_Z], ctx->f64[B200SPH_H], ctx->perm, ctx->skey,
-            ctx->n_sorted, ctx->G, ctx->A0, ctx->A, ctx->AB, ctx->red_u32);
+            ctx->n_sorted, ctx->G, ctx->A0, ctx->A, ctx->AB, ctx->R, ctx->red_u32);
         LAUNCH_CHECK();
     }
     ctx->drift_measured = false;
@@ -1578,7 +1594,7 @@ int b200sph_nnps_update(b200sph_ctx *ctx)
         k_canon<<<ns, 256, 0, ctx->stream>>>(ctx->perm_tmp, ctx->key_of, ctx->cell_start, ntot, ctx->perm, ctx->skey, ctx->rank);
         LAUNCH_CHECK();
         k_pack_pos<<<ns, 256, 0, ctx->stream>>>(ctx->f64[B200SPH_X], ctx->f64[B200SPH_Y], ctx->f64[B200SPH_Z], ctx->f64[B200SPH_H],
-                                                ctx->perm, ctx->skey, ntot, G, ctx->A, ctx->AB, ctx->ptype, ctx->stype);
+                                                ctx->perm, ctx->skey, ntot, G, ctx->A, ctx->AB, ctx->ptype, ctx->stype, ctx->R);
         LAUNCH_CHECK();
         if (use_lists)
             CU(cudaMemcpyAsync(ctx->A0, ctx->A, 16 * (size_t)ntot, cudaMemcpyDeviceToDevice, ctx->stream));
@@ -1732,7 +1748,7 @@ static int pack_state(b200sph_ctx *ctx)
         k_pack_state<<<(unsigned)cdiv(ctx->n_sorted, 256), 256, 0, ctx->stream>>>(
             ctx->f64[B200SPH_U], ctx->f64[B200SPH_V], ctx->f64[B200SPH_W], ctx->f64[B200SPH_M], ctx->f64[B200SPH_RHO],
             ctx->f32[B200SPH_P - N_F64], ctx->f32[B200SPH_CS - N_F64], ctx->ptype, ctx->perm, ctx->n_sorted, ctx->B, ctx->C, ctx->AB,
-            ctx->eos_pending, ctx->eos_any ? 1 : 0);
+            ctx->eos_pending, ctx->eos_any ? 1 : 0, ctx->R, ctx->r32_cls);
         LAUNCH_CHECK();
         memset(ctx->eos_pending.on, 0, sizeof(ctx->eos_pending.on));
         ctx->eos_any = false;
@@ -1825,7 +1841,8 @@ int b200sph_ferrari_h(b200sph_ctx *ctx, int arr, double hdx, int dim, int real_o
         LAUNCH_CHECK();
     }
     ctx->domain_valid = false;  // h changed: the next update_domain must re-reduce it
-    ctx->h_dirty = true;
+    ctx->h_dirty = ctx->uni_dirty = true;
+    ctx->hm_static = false;     // and keeps changing: no uniform-h kernel from here on
     ctx->grid_valid = false, ctx->packed_valid = false;
     return 0;
 }
@@ -1979,7 +1996,8 @@ int b200sph_generic_launch(b200sph_ctx *ctx, int module, const char *kernel, int
     // what was derived from the properties the bodies stored to is stale
     if (writes & 1) {
         ctx->grid_valid = false, ctx->packed_valid = false;
-        ctx->domain_valid = false, ctx->h_dirty = true;
+        ctx->domain_valid = false, ctx->h_dirty = ctx->uni_dirty = true;
+        ctx->hm_static = false;
     }
     if (writes & 2) ctx->state_packed = false, ctx->spec_records = false;
     return 0;
@@ -1995,6 +2013,109 @@ int b200sph_set_dest_range(b200sph_ctx *ctx, int arr, int64_t start, int64_t sto
     ctx->dst_hi[arr] = stop;
     ctx->dst_ranged = true;
     return 0;
+}
+
+int b200sph_set_hm_static(b200sph_ctx *ctx, int on)
+{
+    ctx->hm_static = on != 0;
+    return 0;
+}
+
+// Whether the WCSPH Group `prog` may run the R32 list kernel, and with what: the sources split
+// into at most two classes of equal equation-mask columns (over the destinations), every class
+// that has an equation for some destination has one m and one Tait EOS (gamma = 7, same rho0
+// and c0, pending for this evaluation: its cs went into the records), one h for every particle,
+// no ghosts.  `lm` is the filter the lists hold entries for; a source the lists can hold is
+// classified even if this Group has no equation for it (its class then has none either).
+// Returns 1 and fills `pa`, 0 to fall back, < 0 on error.  Only a change of h or m costs a device
+// reduction (uni_dirty); the rest is a few loops over the 8 x 8 equation masks per pass.
+struct R32Plan {
+    unsigned cls;       // bit a: array a is source class 1
+    int rep[2];         // PairArgs.r32_*
+    float m[2], coef[2];
+};
+static int r32_plan(b200sph_ctx *ctx, const b200sph_pair_program *prog, const unsigned long long *lm, R32Plan &pa)
+{
+    bool dest[B200SPH_MAX_ARRAYS];
+    for (int d = 0; d < ctx->narr; d++) {
+        dest[d] = false;
+        for (int sx = 0; sx < ctx->narr; sx++)
+            if (prog->eqmask[d][sx]) dest[d] = true;
+    }
+    if (!ctx->pair_r32 || !ctx->hm_static || !ctx->eos_any) return 0;
+    if (ctx->mirror[0] || ctx->mirror[1] || ctx->mirror[2] || ctx->peer_connected) return 0;
+    for (int a = 0; a < ctx->narr; a++)
+        if (ctx->arr[a].n != ctx->arr[a].n_real) return 0;
+    if (ctx->uni_dirty) {
+        if (!ctx->uni_red) CU(cudaMalloc((void **)&ctx->uni_red, 4 * B200SPH_MAX_ARRAYS * sizeof(long long)));
+        long long init[4 * B200SPH_MAX_ARRAYS];
+        for (int k = 0; k < 4 * B200SPH_MAX_ARRAYS; k++) init[k] = d2o(1e300);
+        CU(cudaMemcpyAsync(ctx->uni_red, init, sizeof(init), cudaMemcpyHostToDevice, ctx->stream));
+        if (ctx->pool_end > 0) {
+            k_uni_minmax<<<(unsigned)cdiv(ctx->pool_end, 256), 256, 0, ctx->stream>>>(
+                ctx->f64[B200SPH_H], ctx->f64[B200SPH_M], ctx->ptype, ctx->pool_end, ctx->uni_red);
+            LAUNCH_CHECK();
+        }
+        CU(cudaMemcpyAsync(init, ctx->uni_red, sizeof(init), cudaMemcpyDeviceToHost, ctx->stream));
+        CU(cudaStreamSynchronize(ctx->stream));
+        for (int a = 0; a < B200SPH_MAX_ARRAYS; a++) {
+            ctx->uni_h[a][0] = o2d(init[4 * a]); ctx->uni_h[a][1] = -o2d(init[4 * a + 1]);
+            ctx->uni_m[a][0] = o2d(init[4 * a + 2]); ctx->uni_m[a][1] = -o2d(init[4 * a + 3]);
+        }
+        ctx->uni_dirty = false;
+    }
+    double h = 0.0;
+    bool have_h = false;
+    for (int a = 0; a < ctx->narr; a++) {
+        if (ctx->arr[a].n == 0) continue;
+        if (ctx->uni_h[a][0] != ctx->uni_h[a][1] || (have_h && ctx->uni_h[a][0] != h)) return 0;
+        h = ctx->uni_h[a][0];
+        have_h = true;
+    }
+    // classes: arrays the lists can hold as sources, by their column of equation bits
+    int rep[2] = {-1, -1}, cl[B200SPH_MAX_ARRAYS];
+    bool used[2] = {false, false};
+    unsigned c1 = 0;
+    for (int sx = 0; sx < ctx->narr; sx++) {
+        cl[sx] = -1;
+        bool listed = false, any = false;
+        for (int d = 0; d < ctx->narr; d++) {
+            if (!dest[d]) continue;   // not a destination of this Group
+            if ((lm[d] >> (8 * sx)) & 0xFFull) listed = true;
+            if (prog->eqmask[d][sx]) any = true;
+        }
+        if (!listed) continue;
+        int c = -1;
+        for (int k = 0; k < 2 && c < 0; k++) {
+            if (rep[k] < 0) { rep[k] = sx; c = k; break; }
+            bool same = true;
+            for (int d = 0; d < ctx->narr; d++)
+                if (dest[d] && prog->eqmask[d][sx] != prog->eqmask[d][rep[k]]) same = false;
+            if (same) c = k;
+        }
+        if (c < 0) return 0;              // a third class
+        if (c == 1) c1 |= 1u << sx;
+        cl[sx] = c;
+        if (!any) continue;               // no equation: m and the EOS do not matter
+        const EosTab &E = ctx->eos_pending;
+        if (!E.on[sx] || E.gamma[sx] != 7.0) return 0;
+        if (ctx->arr[sx].n > 0 && ctx->uni_m[sx][0] != ctx->uni_m[sx][1]) return 0;
+        const float m = (float)ctx->uni_m[sx][0];
+        const float coef = (float)(E.c0[sx] / (E.rho0[sx] * E.rho0[sx] * E.rho0[sx]));
+        if (used[c] && pa.m[c] != m) return 0;
+        // the members of a class share their column, so all of them have equations here
+        for (int t = 0; t < sx; t++)
+            if (cl[t] == c && (E.rho0[t] != E.rho0[sx] || E.c0[t] != E.c0[sx])) return 0;
+        pa.m[c] = m;
+        pa.coef[c] = coef;
+        used[c] = true;
+    }
+    for (int c = 0; c < 2; c++)
+        if (!used[c]) pa.m[c] = pa.coef[c] = 0.f;
+    pa.rep[0] = rep[0] < 0 ? 0 : rep[0];
+    pa.rep[1] = rep[1] < 0 ? pa.rep[0] : rep[1];
+    pa.cls = c1;
+    return 1;
 }
 
 int b200sph_pair_pass(b200sph_ctx *ctx, const b200sph_pair_program *prog, int64_t *pairs_out)
@@ -2037,6 +2158,25 @@ int b200sph_pair_pass(b200sph_ctx *ctx, const b200sph_pair_program *prog, int64_
             if (d < ctx->narr && sx < ctx->narr && prog->eqmask[d][sx]) want[d] |= 0xFFull << (8 * sx);
     }
     if (use_lists && ctx->lists_valid && !lists_cover(ctx, want)) ctx->lists_valid = false;
+    // the WCSPH scheme's Group (continuity + momentum + XSPH, no tensile correction) has a
+    // leaner kernel variant (B200SPH_PAIR_SPEC=0: always the generic one) ...
+    unsigned prog_bits = 0;
+    for (int d = 0; d < ctx->narr; d++)
+        for (int sx = 0; sx < ctx->narr; sx++) prog_bits |= prog->eqmask[d][sx];
+    const bool wcsph_only = ctx->pair_spec && !(prog_bits & ~(unsigned)PAIR_EQS_WCSPH) && !prog->tensile_correction;
+    // ... and that one a 32-byte-record form (r32_plan); a new class split re-packs the state
+    // records (the sign of rho in R)
+    R32Plan r32p;
+    int r32 = 0;
+    if (use_lists && !ranged && wcsph_only) {
+        unsigned long long lm[B200SPH_MAX_ARRAYS];
+        for (int d = 0; d < B200SPH_MAX_ARRAYS; d++) lm[d] = ctx->list_mask[d] | want[d];   // what build_lists keeps
+        if ((r32 = r32_plan(ctx, prog, lm, r32p)) < 0) return r32;
+        if (r32 && r32p.cls != ctx->r32_cls) {
+            ctx->r32_cls = r32p.cls;
+            ctx->state_packed = false;
+        }
+    }
     // the peer protocol's refresh is still in flight and every record a ghost-free CTA
     // reads is in place: those CTAs go first, the main stream waits for the halo only then
     const bool overlap = ctx->comm_pending && use_lists && ctx->lists_valid && ctx->chunks_valid && ctx->state_packed &&
@@ -2088,12 +2228,10 @@ int b200sph_pair_pass(b200sph_ctx *ctx, const b200sph_pair_program *prog, int64_
     pa.nu4 = (float)(4.0 * prog->nu); pa.eta = (float)prog->eta;
     pa.tensile = prog->tensile_correction;
     pa.real_only = prog->real_only;
-    // the WCSPH scheme's Group (continuity + momentum + XSPH, no tensile correction) has a
-    // leaner kernel variant (B200SPH_PAIR_SPEC=0: always the generic one)
-    unsigned prog_bits = 0;
-    for (int d = 0; d < ctx->narr; d++)
-        for (int sx = 0; sx < ctx->narr; sx++) prog_bits |= prog->eqmask[d][sx];
-    const bool wcsph_only = ctx->pair_spec && !(prog_bits & ~(unsigned)PAIR_EQS_WCSPH) && !prog->tensile_correction;
+    if (r32) {
+        pa.R = ctx->R;
+        for (int c = 0; c < 2; c++) pa.r32_rep[c] = r32p.rep[c], pa.r32_m[c] = r32p.m[c], pa.r32_coef[c] = r32p.coef[c];
+    }
     if (ranged)
         for (int d = 0; d < ctx->narr; d++) {
             pa.doff[d] = ctx->arr[d].off;
@@ -2127,9 +2265,12 @@ int b200sph_pair_pass(b200sph_ctx *ctx, const b200sph_pair_program *prog, int64_
             if (overlap && phase == 0 && ctx->push_first) CU(cudaStreamWaitEvent(ctx->stream, ctx->ev_pushed, 0));
             switch (ctx->kernel * 4 + ctx->dim) {
 #define LIST_LAUNCH(K, D, M, Q) k_pair_list<K, D, M, Q><<<nb, LIST_NT, 0, lst_stream>>>(pa, ctx->cnt, ctx->lst, ctx->capg, ids)
+#define LIST_LAUNCH_R32(K, D, M) k_pair_list<K, D, M, PAIR_EQS_WCSPH, false, true><<<nb, LIST_NT, 0, lst_stream>>>(pa, ctx->cnt, ctx->lst, ctx->capg, ids)
 #define LIST_CASE(K, D)                                                          \
     case K * 4 + D:                                                              \
         if (ranged) k_pair_list<K, D, 6, PAIR_EQS_ALL, true><<<nb, LIST_NT, 0, lst_stream>>>(pa, ctx->cnt, ctx->lst, ctx->capg, ids); \
+        else if (r32 && ctx->pair_minb_r32 >= 8) LIST_LAUNCH_R32(K, D, 8);          \
+        else if (r32) LIST_LAUNCH_R32(K, D, 7);                                    \
         else if (wcsph_only && ctx->pair_minb >= 8) LIST_LAUNCH(K, D, 8, PAIR_EQS_WCSPH); \
         else if (wcsph_only && ctx->pair_minb == 7) LIST_LAUNCH(K, D, 7, PAIR_EQS_WCSPH); \
         else if (ctx->pair_minb >= 7) LIST_LAUNCH(K, D, 7, PAIR_EQS_ALL);          \
@@ -2138,6 +2279,7 @@ int b200sph_pair_pass(b200sph_ctx *ctx, const b200sph_pair_program *prog, int64_
                 LIST_CASE(0, 1) LIST_CASE(0, 2) LIST_CASE(0, 3) LIST_CASE(1, 2) LIST_CASE(1, 3)
                 LIST_CASE(2, 1) LIST_CASE(2, 2) LIST_CASE(2, 3) LIST_CASE(3, 1) LIST_CASE(3, 2) LIST_CASE(3, 3)
 #undef LIST_LAUNCH
+#undef LIST_LAUNCH_R32
 #undef LIST_CASE
             default: return set_err(ctx, "pair_pass: unsupported kernel/dim combination");
             }
@@ -2156,6 +2298,7 @@ int b200sph_pair_pass(b200sph_ctx *ctx, const b200sph_pair_program *prog, int64_
             }
         }
         ctx->stats.pair_launches++;
+        if (r32) ctx->n_pair_r32++;
     } else if (ctx->n_sorted > 0) {
         const unsigned nb = (unsigned)cdiv(ctx->n_sorted, PAIR_WARPS * PAIR_CHUNK);
         switch (ctx->kernel) {
@@ -2528,6 +2671,7 @@ static int stage_impl(b200sph_ctx *ctx, int arr, int which, double dt, bool devd
         q.p = ctx->f32[B200SPH_P - N_F64]; q.cs = ctx->f32[B200SPH_CS - N_F64];
         q.rank = ctx->rank; q.key_of = ctx->key_of;
         q.A0 = ctx->A0; q.AB = ctx->AB; q.C = ctx->C;
+        q.R = ctx->R; q.r32_cls = ctx->r32_cls;
         q.G = ctx->G;
         q.red_u32 = ctx->red_u32;
         q.dt_cfl = ctx->f32[B200SPH_DT_CFL - N_F64]; q.dt_force = ctx->f32[B200SPH_DT_FORCE - N_F64];
@@ -2829,7 +2973,7 @@ static int mirror_create(b200sph_ctx *ctx)
     ctx->ptype_dirty = true;
     ctx->grid_valid = false, ctx->packed_valid = false;
     ctx->topo_dirty = true;
-    ctx->h_dirty = true;
+    ctx->h_dirty = ctx->uni_dirty = true;
     ctx->domain_valid = false;
     ctx->state_packed = false;
     return 0;
@@ -2934,7 +3078,7 @@ int b200sph_halo_append(b200sph_ctx *ctx, int arr, const double *dev_buf, int64_
     ctx->ptype_dirty = true;
     ctx->grid_valid = false, ctx->packed_valid = false;
     ctx->topo_dirty = true;
-    ctx->h_dirty = true;
+    ctx->h_dirty = ctx->uni_dirty = true;
     ctx->domain_valid = false;
     ctx->state_packed = false;
     return 0;
@@ -2991,7 +3135,7 @@ int b200sph_nnps_drift(b200sph_ctx *ctx, double out[2])
         CU(cudaMemsetAsync(ctx->red_u32, 0, 2 * sizeof(unsigned), ctx->stream));
         k_pack_pos_light<<<(unsigned)cdiv(ctx->n_sorted, 256), 256, 0, ctx->stream>>>(
             ctx->f64[B200SPH_X], ctx->f64[B200SPH_Y], ctx->f64[B200SPH_Z], ctx->f64[B200SPH_H], ctx->perm, ctx->skey,
-            ctx->n_sorted, ctx->G, ctx->A0, ctx->A, ctx->AB, ctx->red_u32);
+            ctx->n_sorted, ctx->G, ctx->A0, ctx->A, ctx->AB, ctx->R, ctx->red_u32);
         LAUNCH_CHECK();
     }
     CU(cudaMemcpyAsync(ctx->red_u32_host, ctx->red_u32, 2 * sizeof(unsigned), cudaMemcpyDeviceToHost, ctx->stream));
@@ -3118,7 +3262,7 @@ int b200sph_nnps_drift_device(b200sph_ctx *ctx, double *dev_ratio)
         CU(cudaMemsetAsync(ctx->red_u32, 0, 2 * sizeof(unsigned), ctx->stream));
         k_pack_pos_light<<<(unsigned)cdiv(ctx->n_sorted, 256), 256, 0, ctx->stream>>>(
             ctx->f64[B200SPH_X], ctx->f64[B200SPH_Y], ctx->f64[B200SPH_Z], ctx->f64[B200SPH_H], ctx->perm, ctx->skey,
-            ctx->n_sorted, ctx->G, ctx->A0, ctx->A, ctx->AB, ctx->red_u32);
+            ctx->n_sorted, ctx->G, ctx->A0, ctx->A, ctx->AB, ctx->R, ctx->red_u32);
         LAUNCH_CHECK();
     }
     k_drift_ratio<<<1, 1, 0, ctx->stream>>>(ctx->red_u32, (float)ctx->radius_scale, (float)ctx->S_abs, dev_ratio);
@@ -3236,7 +3380,7 @@ int b200sph_peer_begin(b200sph_ctx *ctx)
         CU(cudaMemsetAsync(ctx->red_u32, 0, 2 * sizeof(unsigned), ctx->stream));
         k_pack_pos_light<<<(unsigned)cdiv(ctx->n_sorted, 256), 256, 0, ctx->stream>>>(
             ctx->f64[B200SPH_X], ctx->f64[B200SPH_Y], ctx->f64[B200SPH_Z], ctx->f64[B200SPH_H], ctx->perm, ctx->skey,
-            ctx->n_sorted, ctx->G, ctx->A0, ctx->A, ctx->AB, ctx->red_u32);
+            ctx->n_sorted, ctx->G, ctx->A0, ctx->A, ctx->AB, ctx->R, ctx->red_u32);
         LAUNCH_CHECK();
     }
     if (!no_build) ctx->packed_valid = true, ctx->drift_measured = true;
@@ -3486,7 +3630,7 @@ int b200sph_drop_ghosts(b200sph_ctx *ctx, int arr)
         ctx->ptype_dirty = true;
         ctx->grid_valid = false, ctx->packed_valid = false;
         ctx->topo_dirty = true;
-        ctx->h_dirty = true;
+        ctx->h_dirty = ctx->uni_dirty = true;
         ctx->state_packed = false;
     }
     return 0;
@@ -3607,7 +3751,7 @@ int b200sph_migrate_out(b200sph_ctx *ctx, int arr, double lo, double hi, double 
     ctx->ptype_dirty = true;
     ctx->grid_valid = false, ctx->packed_valid = false;
     ctx->topo_dirty = true;
-    ctx->h_dirty = true;
+    ctx->h_dirty = ctx->uni_dirty = true;
     ctx->domain_valid = false;
     ctx->state_packed = false;
     return 0;
@@ -3663,8 +3807,15 @@ int b200sph_get_stats(b200sph_ctx *ctx, b200sph_stats *out)
     *out = ctx->stats;
     return 0;
 }
+int b200sph_get_pair_r32_launches(b200sph_ctx *ctx, int64_t *out)
+{
+    *out = ctx->n_pair_r32;
+    return 0;
+}
+
 int b200sph_reset_stats(b200sph_ctx *ctx)
 {
+    ctx->n_pair_r32 = 0;
     b200sph_stats tmp;
     b200sph_get_stats(ctx, &tmp);  // drain pending events
     memset(&ctx->stats, 0, sizeof(ctx->stats));

@@ -64,7 +64,8 @@ __global__ void k_pack_pos(const double *__restrict__ x, const double *__restric
                            const double *__restrict__ z, const double *__restrict__ h,
                            const uint32_t *__restrict__ perm, const uint32_t *__restrict__ skey,
                            long long n, GridDev G, float4 *__restrict__ A, float4 *__restrict__ AB,
-                           const uint8_t *__restrict__ ptype, uint8_t *__restrict__ stype)
+                           const uint8_t *__restrict__ ptype, uint8_t *__restrict__ stype,
+                           float4 *__restrict__ R = nullptr)
 {
     long long s = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (s >= n) return;
@@ -80,17 +81,24 @@ __global__ void k_pack_pos(const double *__restrict__ x, const double *__restric
     a.w = (float)h[g];
     A[s] = a;
     AB[2 * s] = a;
+    if (R) {   // the position half of the 32-byte source record (PairArgs.R)
+        float *r = reinterpret_cast<float *>(R + 2 * s);
+        r[0] = a.x; r[1] = a.y; r[2] = a.z;
+    }
 }
 
 // B[s] = (u, v, w, m);  C[s] = (rho, p/rho^2, cs, type); pending TaitEOS /
-// TaitEOSHGCorrection calls (wc/basic.py:60-65,118-126) are applied on the way
+// TaitEOSHGCorrection calls (wc/basic.py:60-65,118-126) are applied on the way.  The state
+// half of the 32-byte source record R (PairArgs.R) goes with them: (rho with the source class
+// in its sign bit, r32_cls bit a = array a is class 1) and (u, v, w, p/rho^2).
 __global__ void k_pack_state(const double *__restrict__ u, const double *__restrict__ v,
                              const double *__restrict__ w, const double *__restrict__ m,
                              double *__restrict__ rho, float *__restrict__ p,
                              float *__restrict__ cs, const uint8_t *__restrict__ ptype,
                              const uint32_t *__restrict__ perm, long long n,
                              float4 *__restrict__ B, float4 *__restrict__ C,
-                             float4 *__restrict__ AB, const EosTab E, const int eos_any)
+                             float4 *__restrict__ AB, const EosTab E, const int eos_any,
+                             float4 *__restrict__ R = nullptr, const unsigned r32_cls = 0)
 {
     long long s = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (s >= n) return;
@@ -125,4 +133,8 @@ __global__ void k_pack_state(const double *__restrict__ u, const double *__restr
     B[s] = b;
     C[s] = c;
     AB[2 * s + 1] = b;
+    if (R) {
+        reinterpret_cast<float *>(R + 2 * s)[3] = __uint_as_float((unsigned)__float_as_int(c.x) | (((r32_cls >> a) & 1u) << 31));
+        R[2 * s + 1] = make_float4(b.x, b.y, b.z, c.y);
+    }
 }

@@ -7,6 +7,15 @@
 // --------------------------------------------------------------------------
 struct PairArgs {
     const float4 *A, *B, *C, *AB;
+    // the 32-byte source records of the R32 variant, two float4 per sorted slot: R[2s] = (x, y, z
+    // cell-relative as in A, +-rho), R[2s+1] = (u, v, w, p / rho^2) -- the fp32 values A / B / C
+    // carry; rho > 0, so its sign bit is free and holds the source class (0 / 1) that stands for
+    // h, m and cs.  Written wherever A / AB / C are written for real particles.
+    const float4 *R;
+    // the R32 variant of k_pair_list: per source class, an array of the class (its byte of
+    // emask gives the class's equation bits), m and cs / rho^3 = c0 / rho0^3
+    int r32_rep[2];
+    float r32_m[2], r32_coef[2];
     const uint32_t *cell_start, *skey, *perm;
     float *arho, *au, *av, *aw, *ax, *ay, *az, *dt_cfl, *dt_force;
     double *rho;  // SummationDensity destination (fp64 state)
@@ -42,14 +51,13 @@ struct Acc {
 #define PAIR_EQS_TENSILE 0x100
 #define PAIR_EQS_ALL 0x1FF
 #define PAIR_EQS_WCSPH (B200SPH_EQ_CONTINUITY | B200SPH_EQ_MOMENTUM | B200SPH_EQ_XSPH)
+// one accepted pair: `bits` are the equations of (destination, source); qv = (x_ij, h_j),
+// Bj = (u, v, w, m)_j, Cj = (rho, p / rho^2, cs)_j
 template <int K, int DIM, int EQS = PAIR_EQS_ALL>
-__device__ __forceinline__ void pair_body(const PairArgs &a, const float4 qv, const float4 Bj,
+__device__ __forceinline__ void pair_eval(const PairArgs &a, const unsigned bits, const float4 qv, const float4 Bj,
                                           const float4 Cj, const float4 Ai, const float4 Bi,
-                                          const float4 Ci, const unsigned long long mask_i,
-                                          const float tmpi, Acc &acc, unsigned &npairs)
+                                          const float4 Ci, const float tmpi, Acc &acc, unsigned &npairs)
 {
-    const int tj = __float_as_int(Cj.w) & 7;
-    const unsigned bits = (unsigned)(mask_i >> (8 * tj)) & (unsigned)(EQS & 0xFF);
     if (!bits) return;
     npairs++;
     const float xij = qv.x, yij = qv.y, zij = qv.z, hj = qv.w;
@@ -121,6 +129,17 @@ __device__ __forceinline__ void pair_body(const PairArgs &a, const float4 qv, co
             acc.az += f * wwij;
         }
     }
+}
+
+template <int K, int DIM, int EQS = PAIR_EQS_ALL>
+__device__ __forceinline__ void pair_body(const PairArgs &a, const float4 qv, const float4 Bj,
+                                          const float4 Cj, const float4 Ai, const float4 Bi,
+                                          const float4 Ci, const unsigned long long mask_i,
+                                          const float tmpi, Acc &acc, unsigned &npairs)
+{
+    const int tj = __float_as_int(Cj.w) & 7;
+    const unsigned bits = (unsigned)(mask_i >> (8 * tj)) & (unsigned)(EQS & 0xFF);
+    pair_eval<K, DIM, EQS>(a, bits, qv, Bj, Cj, Ai, Bi, Ci, tmpi, acc, npairs);
 }
 
 template <int K, int DIM>

@@ -273,7 +273,37 @@ __device__ __forceinline__ void pair_entry(const PairArgs &a, const bool live, c
         pair_body<K, DIM, EQS>(a, make_float4(xij, yij, zij, Aj.w), Bj, Cj, Ai, Bi, Ci, mask_i, Ci.y, acc, npairs);
 }
 
-template <int K, int DIM, int MINB, int EQS, bool RANGED = false>
+// The same entry from the 32-byte record R (the R32 variant: one h for every particle, m and
+// the Tait EOS uniform within each of at most two source classes, no ghosts).  h_j = h_i makes
+// the two-sided accept test one-sided; the sign bit of rho_j selects the class: its equation
+// bits, m_j, and cs_j = c0 (rho_j / rho0)^3 recomputed in fp32 (the only arithmetic that differs
+// from the 48-byte path: a few ulp of cs_j inside Pi_ij).
+template <int K, int DIM, int EQS>
+__device__ __forceinline__ void pair_entry_r32(const PairArgs &a, const bool live, const uint32_t e,
+                                               const float4 Pj, const float4 Qj, const float4 Ai,
+                                               const float4 Bi, const float4 Ci, const float hi2,
+                                               const unsigned bits0, const unsigned bits1,
+                                               Acc &acc, unsigned &npairs)
+{
+    const float dxc = __uint_as_float((e & 3u) | 0x4B000000u) - 8388609.0f;
+    const float dyc = __uint_as_float(((e >> 2) & 3u) | 0x4B000000u) - 8388609.0f;
+    const float dzc = __uint_as_float(((e >> 4) & 3u) | 0x4B000000u) - 8388609.0f;
+    const float xij = fmaf(-dxc, a.cellx, Ai.x - Pj.x), yij = fmaf(-dyc, a.celly, Ai.y - Pj.y),
+                zij = fmaf(-dzc, a.cellz, Ai.z - Pj.z);
+    const float r2 = xij * xij + yij * yij + zij * zij;
+    if (live && r2 < hi2) {
+        const bool c1 = __float_as_int(Pj.w) < 0;
+        const float rhoj = fabsf(Pj.w);
+        const float csj = (c1 ? a.r32_coef[1] : a.r32_coef[0]) * (rhoj * rhoj * rhoj);
+        pair_eval<K, DIM, EQS>(a, c1 ? bits1 : bits0, make_float4(xij, yij, zij, Ai.w),
+                               make_float4(Qj.x, Qj.y, Qj.z, c1 ? a.r32_m[1] : a.r32_m[0]),
+                               make_float4(rhoj, Qj.w, csj, 0.f), Ai, Bi, Ci, Ci.y, acc, npairs);
+    }
+}
+
+// R32: the sources come from the 32-byte records R (pair_entry_r32); the destination still
+// reads its own A / B / C, once and coalesced
+template <int K, int DIM, int MINB, int EQS, bool RANGED = false, bool R32 = false>
 __global__ void __launch_bounds__(LIST_NT, MINB) k_pair_list(const PairArgs a, const uint32_t *__restrict__ cnt,
                                                             const uint32_t *__restrict__ lst, const int capg,
                                                             const uint32_t *__restrict__ chunk_ids)
@@ -308,12 +338,23 @@ __global__ void __launch_bounds__(LIST_NT, MINB) k_pair_list(const PairArgs a, c
     const float hi2 = a.k2 * Ai.w * Ai.w;
     Acc acc = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
     unsigned npairs = 0;
-    struct Rec { float4 A, B, C; };
-    list_walk<Rec>(nxt, count, cmax,
-        [&](const uint32_t e, Rec &r) { ld_rec(a, e, r.A, r.B, r.C); },
-        [&](const bool live, const uint32_t e, const Rec &r) {
-            pair_entry<K, DIM, EQS>(a, live, e, r.A, r.B, r.C, Ai, Bi, Ci, hi2, mask_i, acc, npairs);
-        });
+    if constexpr (R32) {
+        const unsigned bits0 = (unsigned)(mask_i >> (8 * a.r32_rep[0])) & (unsigned)(EQS & 0xFF);
+        const unsigned bits1 = (unsigned)(mask_i >> (8 * a.r32_rep[1])) & (unsigned)(EQS & 0xFF);
+        struct Rec { float4 P, Q; };
+        list_walk<Rec>(nxt, count, cmax,
+            [&](const uint32_t e, Rec &r) { ld_256(a.R + 2u * LIST_J(e), r.P, r.Q); },
+            [&](const bool live, const uint32_t e, const Rec &r) {
+                pair_entry_r32<K, DIM, EQS>(a, live, e, r.P, r.Q, Ai, Bi, Ci, hi2, bits0, bits1, acc, npairs);
+            });
+    } else {
+        struct Rec { float4 A, B, C; };
+        list_walk<Rec>(nxt, count, cmax,
+            [&](const uint32_t e, Rec &r) { ld_rec(a, e, r.A, r.B, r.C); },
+            [&](const bool live, const uint32_t e, const Rec &r) {
+                pair_entry<K, DIM, EQS>(a, live, e, r.A, r.B, r.C, Ai, Bi, Ci, hi2, mask_i, acc, npairs);
+            });
+    }
     if (active) {
         unsigned all_bits = 0;
 #pragma unroll

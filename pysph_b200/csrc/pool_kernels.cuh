@@ -202,6 +202,8 @@ struct FusePackArgs {
     const uint32_t *rank, *key_of;   // pool index -> sorted slot / cell key of the current build
     const float4 *A0;                // packed positions at build time (sorted order)
     float4 *AB, *C;
+    float4 *R;                       // the 32-byte source records (PairArgs.R)
+    unsigned r32_cls;                // bit a: array a is source class 1
     GridDev G;
     unsigned *red_u32;
     const float *dt_cfl, *dt_force;
@@ -285,6 +287,8 @@ __global__ void __launch_bounds__(256, 5) k_stage_pack(const StageArgs a, const 
             q.AB[2 * (size_t)s] = A;
             q.AB[2 * (size_t)s + 1] = B;
             q.C[s] = C;
+            q.R[2 * (size_t)s] = make_float4(A.x, A.y, A.z, __uint_as_float((unsigned)__float_as_int(C.x) | (((q.r32_cls >> ar) & 1u) << 31)));
+            q.R[2 * (size_t)s + 1] = make_float4(B.x, B.y, B.z, C.y);
             const float4 b0 = q.A0[s];
             const float ex = A.x - b0.x, ey = A.y - b0.y, ez = A.z - b0.z;
             d2 = ex * ex + ey * ey + ez * ez;
@@ -413,4 +417,36 @@ __global__ void k_f32_to_f64(const float *__restrict__ in, double *__restrict__ 
 {
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) out[i] = (double)in[i];
+}
+
+// per array (min, max) of h and of m over the real particles, as ordered int64 (d2o):
+// out[4 a + 0 / 1] = min h / -max h, out[4 a + 2 / 3] = min m / -max m (everything a minimum,
+// so that one initial value serves every slot).  Decides whether the R32 list kernel applies.
+__global__ void k_uni_minmax(const double *__restrict__ h, const double *__restrict__ m,
+                             const uint8_t *__restrict__ ptype, long long pool_end, long long *__restrict__ out)
+{
+    const unsigned FULL = 0xffffffffu;
+    const long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const uint8_t t = g < pool_end ? ptype[g] : (uint8_t)PT_INVALID;
+    const bool valid = t != PT_INVALID && !(t & PT_GHOST);
+    double v[4] = {1e300, 1e300, 1e300, 1e300};
+    if (valid) {
+        v[0] = h[g]; v[1] = -v[0];
+        v[2] = m[g]; v[3] = -v[2];
+    }
+    // pools are array after array: a warp almost always holds one array, reduce it first
+    const int arr = valid ? (t & 7) : -1;
+    const int arr0 = __shfl_sync(FULL, arr, 0);
+    const bool one = __ballot_sync(FULL, arr == arr0 || arr < 0) == FULL;
+    if (one) {
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1)
+#pragma unroll
+            for (int k = 0; k < 4; k++) v[k] = fmin(v[k], __shfl_xor_sync(FULL, v[k], o));
+    }
+    if (one ? ((threadIdx.x & 31) == 0 && arr0 >= 0) : valid) {
+        long long *o = out + 4 * (one ? arr0 : arr);
+#pragma unroll
+        for (int k = 0; k < 4; k++) atomicMin(o + k, d2o(v[k]));
+    }
 }

@@ -396,7 +396,7 @@ __global__ void k_pack_pos_light(const double *__restrict__ x, const double *__r
                                  const uint32_t *__restrict__ perm, const uint32_t *__restrict__ skey,
                                  long long n, GridDev G, const float4 *__restrict__ A0,
                                  float4 *__restrict__ A, float4 *__restrict__ AB,
-                                 unsigned *__restrict__ red_u32)
+                                 float4 *__restrict__ R, unsigned *__restrict__ red_u32)
 {
     long long s = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     float d2 = 0.f, dh = 0.f;
@@ -412,6 +412,8 @@ __global__ void k_pack_pos_light(const double *__restrict__ x, const double *__r
         a.w = (float)h[g];
         A[s] = a;
         AB[2 * s] = a;
+        float *r = reinterpret_cast<float *>(R + 2 * s);   // the 32-byte source record (PairArgs.R)
+        r[0] = a.x; r[1] = a.y; r[2] = a.z;
         const float4 b = A0[s];
         const float dx = a.x - b.x, dy = a.y - b.y, dz = a.z - b.z;
         d2 = dx * dx + dy * dy + dz * dz;
